@@ -49,6 +49,8 @@ CONFIG_NAMES = {
           '200x200, 10 waypoints, xyz + quaternion + gripper heads)',
     'c5': 'C5: Grasp2Vec train step (scene + goal truncated ResNet-50 towers, n-pairs loss) on 224x224 triples',
 }
+# --dump-outputs: at most 4 Mi float32 elements per array, 64 MB over the three arrays a step writes
+DUMP_MAX_ELEMENTS = 1 << 22
 
 
 def parse_args():
@@ -69,7 +71,13 @@ def parse_args():
   p.add_argument('--no-cpu-baseline', action='store_true')
   p.add_argument('--no-e2e', action='store_true')
   p.add_argument('--no-extras', action='store_true', help='skip the Grasping44 / CEM side measurements of c2')
+  p.add_argument('--dump-outputs', metavar='DIR', default=None,
+                 help='after the timed steps, write what the last timed step computed (its loss, the trainable variables '
+                      'and the moving statistics it updated) as DIR/<name>.npy in float32; an array of more than %d '
+                      'elements is replaced by the elements at a fixed, seeded sample of its indices' % DUMP_MAX_ELEMENTS)
   args = p.parse_args()
+  if args.dump_outputs and args.impl != 'b200':
+    p.error('--dump-outputs writes the outputs of the b200 engine')
   if args.batch is None:
     args.batch = 512 if args.config in ('c2', 'c3') else 256
   return args
@@ -372,6 +380,20 @@ def timed_steps(rt, fn, steps, warmup, profile=True, sample_clocks=False):
   return rt.max_over_ranks(ev0.elapsed_time(ev1)) / steps, out, prof, int(launches), clocks
 
 
+def dump_outputs(args, rt, loss, vs):
+  """--dump-outputs: the loss the last timed step returned and the variables it left behind (trainable, then moving
+  statistics), as float32 .npy files.  Equal arguments give equal inputs, so two builds can be compared file by file.
+  Larger arrays keep the elements at the same RandomState(0) sample of indices in every run."""
+  if not args.dump_outputs or rt.rank != 0:
+    return
+  os.makedirs(args.dump_outputs, exist_ok=True)
+  for name, t in (('loss', loss), ('trainable_variables', vs.flat), ('moving_statistics', vs.state_flat)):
+    a = t.detach().float().cpu().numpy()
+    if a.size > DUMP_MAX_ELEMENTS:
+      a = a.reshape(-1)[np.sort(np.random.RandomState(0).choice(a.size, DUMP_MAX_ELEMENTS, replace=False))]
+    np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
+
+
 def conv_roofline(prof, elapsed_ms_total, steps, rank):
   by_kind, by_shape = {}, {}
   peaks = measured_peaks()
@@ -617,6 +639,7 @@ def run_critic(args, rt):
   step.build(*sets[0][:2])
   ms, loss, prof, launches, clocks = timed_steps(rt, lambda i: step.step(*sets[i % 2]), args.steps, args.warmup,
                                                  sample_clocks=True)
+  dump_outputs(args, rt, loss, step.vs)
   loss_value = float(loss)
   roofline = conv_roofline(prof, ms * args.steps, args.steps, rt.rank)
   value = b * rt.world * 1000.0 / ms
@@ -745,6 +768,7 @@ def run_t2r(args, rt):
     return model.train_step(features, labels)
 
   ms, loss, prof, launches, clocks = timed_steps(rt, one, args.steps, args.warmup, sample_clocks=True)
+  dump_outputs(args, rt, loss, model.variable_store)
   roofline = conv_roofline(prof, ms * args.steps, args.steps, rt.rank)
   value = args.batch * rt.world * 1000.0 / ms
   extra = {'loss': float(loss), 'peak_mem_gb': torch.cuda.max_memory_allocated(rt.dev) / 1e9,
@@ -762,6 +786,13 @@ def run_t2r(args, rt):
 
 
 def run_b200(args):
+  from tensor2robot_b200.preprocessors import image_transformations
+  # the c4 / c5 batches and the e2e host batches come from make_random_numpy (global NumPy RNG), the training crops
+  # and photometric draws from image_transformations: seeded (per rank) so that equal arguments give equal inputs in
+  # every run
+  rank = int(os.environ.get('RANK', '0'))
+  np.random.seed(rank)
+  image_transformations.seed(rank)
   rt = Runtime(args)
   if args.config in ('c2', 'c3'):
     ms, value, roofline, launches, clocks, e2e, extra = run_critic(args, rt)

@@ -4,11 +4,20 @@ oracle (oracle/vision_layers.py) cross-checked against independent restatements.
 import os
 
 import numpy as np
+import pytest
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 FIXTURE = os.path.join(HERE, 'golden', 'pose_env_test_data.tfrecord')
 GOLDEN = np.load(os.path.join(HERE, 'golden', 'pose_env_golden.npz'))
+
+
+@pytest.fixture(autouse=True)
+def _host_image_decoder(monkeypatch):
+  """The host decoder (numpy out) on every machine: 'auto' picks the device decoder where a GPU is present, and
+  tests/test_jpeg.py checks that one against this one."""
+  from tensor2robot_b200.utils import tfdata
+  monkeypatch.setattr(tfdata, 'IMAGE_DECODER', 'host')
 
 
 def test_model_specs():

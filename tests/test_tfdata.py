@@ -26,6 +26,13 @@ GOLDEN = np.load(os.path.join(HERE, 'golden', 'pose_env_golden.npz'))
 TSPEC = utils.ExtendedTensorSpec
 
 
+@pytest.fixture(autouse=True)
+def _host_image_decoder(monkeypatch):
+  """The host decoder (numpy out) on every machine: 'auto' picks the device decoder where a GPU is present, and
+  tests/test_jpeg.py checks that one against this one."""
+  monkeypatch.setattr(tfdata, 'IMAGE_DECODER', 'host')
+
+
 def test_library_exports_every_declared_symbol():
   lib = _lib.lib()
   header = open(os.path.join(os.path.dirname(HERE), 'include', 't2r_b200.h')).read()
