@@ -106,6 +106,28 @@ int32_t t2r_conv2d_wgrad_bnrelu(const T2RConvDesc* d, const void* x_raw, const f
 int32_t t2r_conv2d_dgrad_bnrelu(const T2RConvDesc* d, const void* dy, const void* w_dgrad, const void* x_raw,
                                 const float* bn_scale, const float* bn_shift, void* g, int32_t accumulate,
                                 double* red, void* stream);
+/* Batch-norm backward through the GEMMs of a 1x1 stride-1 unpadded consumer y = conv1x1(z, w), z = relu(scale*x +
+ * shift), m = [scale*x + shift > 0], g = m * conv_transpose(dy, w).  Three launches replace the data gradient, the
+ * reduction pass and the apply pass:
+ *   wgrad_bnsums      : dw += dy^T * z as scale * P + shift * Q with P = dy^T (m*x), Q = dy^T m (one MMA yields both),
+ *                       and sums[c] += sum_n w[n, c] * Q[n, c] (= sum g), sums[Cin + c] += sum_n w[n, c] * P[n, c]
+ *                       (= sum g*x); sums fp64 [2*Cin], caller zeroes; w_dgrad is the bf16 [Cin][Cout] copy the data
+ *                       gradient multiplies with.
+ *   bn_backward_gemm_finalize : dgamma / dbeta (written) and coef = [kb | kc] fp32 [2*C], the per-channel
+ *                       coefficients of dx = scale*g + kb*x + kc.
+ *   dgrad_bnapply     : dx = scale * m * conv_transpose(dy, w) + kb*x + kc (+ dpass, may be null) in the epilogue of
+ *                       the TMA data-gradient kernel, from the fp32 accumulator; g is never written.
+ * dgrad_bnapply_supported(d) returns 1 when d is such a convolution and its data gradient runs on the TMA-epilogue
+ * kernel (Cin <= 128, or a multiple of 256 with Cout <= 256); dgrad_bnapply fails with T2R_ERR_ARG otherwise. */
+int32_t t2r_conv2d_wgrad_bnsums(const T2RConvDesc* d, const void* x_raw, const float* bn_scale, const float* bn_shift,
+                                const void* dy, const void* w_dgrad, float* dw, double* sums, void* stream);
+int32_t t2r_bn_backward_gemm_finalize(const double* sums, int64_t rows, int32_t C, const float* mean,
+                                      const float* invstd, const float* scale, float* dgamma, float* dbeta,
+                                      float* coef, void* stream);
+int32_t t2r_conv2d_dgrad_bnapply_supported(const T2RConvDesc* d);
+int32_t t2r_conv2d_dgrad_bnapply(const T2RConvDesc* d, const void* dy, const void* w_dgrad, const void* x_raw,
+                                 const float* bn_scale, const float* bn_shift, const float* coef, const void* dpass,
+                                 void* dx, void* stream);
 /* ---- high-precision PREDICT path (csrc/hp.cu) ----------------------------------------------
  * fp32 activations; a convolution y = conv(x, w) is evaluated as bf16x3: x3 = [hi | lo | hi] (t2r_hp_split3), w3 =
  * [w_hi | w_hi | w_lo] (t2r_hp_pack_weights3), then t2r_conv2d_fprop with Cin' = 3*Cin and T2R_EPI_OUT_F32 (fp32

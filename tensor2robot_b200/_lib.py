@@ -75,6 +75,10 @@ _PROTOS = {
     't2r_conv2d_fprop_bnrelu': (_I32, [_CD, _P, _P, _P, _P, _P, _P, _P, _P]),
     't2r_conv2d_wgrad_bnrelu': (_I32, [_CD, _P, _P, _P, _P, _P, _P]),
     't2r_conv2d_dgrad_bnrelu': (_I32, [_CD, _P, _P, _P, _P, _P, _P, _I32, _P, _P]),
+    't2r_conv2d_wgrad_bnsums': (_I32, [_CD, _P, _P, _P, _P, _P, _P, _P, _P]),
+    't2r_conv2d_dgrad_bnapply_supported': (_I32, [_CD]),
+    't2r_conv2d_dgrad_bnapply': (_I32, [_CD, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    't2r_bn_backward_gemm_finalize': (_I32, [_P, _I64, _I32, _P, _P, _P, _P, _P, _P, _P]),
     't2r_pack_weights': (_I32, [_P, _P, _P, _I32, _I32, _I32, _P]),
     't2r_hp_split3': (_I32, [_P, _P, _I64, _I32, _P]),
     't2r_hp_pack_weights3': (_I32, [_P, _P, _I32, _I32, _I32, _P]),
@@ -166,7 +170,8 @@ _PROTOS = {
 }
 
 # Functions whose int return value is a status code (checked by `call`).
-_STATUS = {n for n, (r, _) in _PROTOS.items() if r is _I32 and n not in ('t2r_version', 't2r_stem_k')}
+_STATUS = {n for n, (r, _) in _PROTOS.items()
+           if r is _I32 and n not in ('t2r_version', 't2r_stem_k', 't2r_conv2d_dgrad_bnapply_supported')}
 
 EXPORTED_SYMBOLS = tuple(sorted(_PROTOS))
 

@@ -30,8 +30,13 @@ constexpr int kMaxStatChannels = 2048;
 //   kProBnRelu (1x1 fprop): the activation tensor map points at the RAW tensor x and four extra warps rewrite
 //              every landed A tile in shared memory as relu(bn_scale * x + bn_shift) before the MMA reads it: the
 //              batch-norm apply pass (bn_apply_rows_kernel) without writing / re-reading z.
+//   kEpiBnApply (1x1 stride-1 data gradients, TMA epilogue only): the batch-norm reduction is already known
+//              (t2r_conv2d_wgrad_bnsums + t2r_bn_backward_gemm_finalize), so the epilogue writes the batch-norm input
+//              gradient directly: dx = bn_scale * [bn_scale * x + bn_shift > 0] * acc + kb * x + kc (+ residual,
+//              the pass-through gradient), bn_coef = [kb | kc].  Neither g nor any column sum is produced.
 constexpr int kEpiBnBwd = 1 << 8;
 constexpr int kProBnRelu = 1 << 9;
+constexpr int kEpiBnApply = 1 << 10;
 
 struct IgemmParams {
   CUtensorMap tmap_a[4];
@@ -52,8 +57,9 @@ struct IgemmParams {
   int flags;
   double* stats;  // optional fp64 [2*Cout]: per-channel sum / sum of squares of the bf16 output (fused bn_stats)
   const void* bn_x;        // kEpiBnBwd: the normalised tensor, addressed like `out`
-  const float* bn_scale;   // kEpiBnBwd: [Cout] of the output view; kProBnRelu: [Cin]
+  const float* bn_scale;   // kEpiBnBwd / kEpiBnApply: [Cout] of the output view; kProBnRelu: [Cin]
   const float* bn_shift;
+  const float* bn_coef;    // kEpiBnApply: fp32 [2 * Cout], kb then kc
 };
 
 // The tap-table kernel with a TMA epilogue (conv_igemm_tma.cu): residual tile in by TMA, output tile

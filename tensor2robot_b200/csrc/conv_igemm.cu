@@ -616,22 +616,44 @@ static int32_t fprop_impl(const T2RConvDesc* d, const void* x, const float* bn_s
 }
 
 static int32_t dgrad_impl(const T2RConvDesc* d, const void* dy, const void* w_dgrad, void* dx, int32_t accumulate,
-                          const void* bn_x, const float* bn_scale, const float* bn_shift, double* red, void* stream);
+                          const void* bn_x, const float* bn_scale, const float* bn_shift, double* red,
+                          const float* bn_coef, const void* dpass, void* stream);
 
 extern "C" int32_t t2r_conv2d_dgrad(const T2RConvDesc* d, const void* dy, const void* w_dgrad,
                                     void* dx, int32_t accumulate, void* stream) {
-  return dgrad_impl(d, dy, w_dgrad, dx, accumulate, nullptr, nullptr, nullptr, nullptr, stream);
+  return dgrad_impl(d, dy, w_dgrad, dx, accumulate, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, stream);
 }
 
 extern "C" int32_t t2r_conv2d_dgrad_bnrelu(const T2RConvDesc* d, const void* dy, const void* w_dgrad,
                                            const void* x_raw, const float* bn_scale, const float* bn_shift, void* g,
                                            int32_t accumulate, double* red, void* stream) {
   T2R_CHECK_ARG(x_raw && bn_scale && bn_shift && red, "conv2d_dgrad_bnrelu: null pointer");
-  return dgrad_impl(d, dy, w_dgrad, g, accumulate, x_raw, bn_scale, bn_shift, red, stream);
+  return dgrad_impl(d, dy, w_dgrad, g, accumulate, x_raw, bn_scale, bn_shift, red, nullptr, nullptr, stream);
+}
+
+extern "C" int32_t t2r_conv2d_dgrad_bnapply_supported(const T2RConvDesc* d) {
+  if (d == nullptr || d->struct_size != sizeof(T2RConvDesc)) return 0;
+  if (d->KH != 1 || d->KW != 1 || d->stride != 1 || d->pad_top != 0 || d->pad_left != 0) return 0;
+  if (d->Cin % 64 != 0 || d->Cout % 64 != 0 || d->Cin <= 0 || d->Cout <= 0) return 0;
+  bool tma = false;
+  pick_block_n(d->Cin, d->Cout, 0, &tma);
+  return tma ? 1 : 0;
+}
+
+extern "C" int32_t t2r_conv2d_dgrad_bnapply(const T2RConvDesc* d, const void* dy, const void* w_dgrad,
+                                            const void* x_raw, const float* bn_scale, const float* bn_shift,
+                                            const float* bn_coef, const void* dpass, void* dx, void* stream) {
+  if (int rc = check_desc(d)) return rc;
+  T2R_CHECK_ARG(x_raw && bn_scale && bn_shift && bn_coef, "conv2d_dgrad_bnapply: null pointer");
+  T2R_CHECK_ARG(t2r_conv2d_dgrad_bnapply_supported(d),
+                "conv2d_dgrad_bnapply: needs a 1x1 stride-1 unpadded convolution whose data gradient runs on the "
+                "TMA-epilogue kernel (Cin <= 128, or a multiple of 256 with Cout <= 256)");
+  return dgrad_impl(d, dy, w_dgrad, dx, 0, x_raw, bn_scale, bn_shift, nullptr, bn_coef, dpass, stream);
 }
 
 static int32_t dgrad_impl(const T2RConvDesc* d, const void* dy, const void* w_dgrad, void* dx, int32_t accumulate,
-                          const void* bn_x, const float* bn_scale, const float* bn_shift, double* red, void* stream) {
+                          const void* bn_x, const float* bn_scale, const float* bn_shift, double* red,
+                          const float* bn_coef, const void* dpass, void* stream) {
   if (int rc = check_desc(d)) return rc;
   T2R_CHECK_ARG(dy && w_dgrad && dx, "null pointer");
   // Batch-norm backward fusion: the epilogues mask and reduce while they write (kEpiBnBwd) unless the launch
@@ -641,7 +663,7 @@ static int32_t dgrad_impl(const T2RConvDesc* d, const void* dy, const void* w_dg
   // memory-bound kernel can afford ~6, e.g. 3.3 ms against 1.1 ms (data gradient) + 1.2 ms (reduction pass) on
   // 512x118x118x256, so the reduction pass below stays the default and the epilogue is opt-in (T2R_BNBWD_EPI=1).
   static const bool epi_bnbwd = std::getenv("T2R_BNBWD_EPI") != nullptr && std::getenv("T2R_BNBWD_EPI")[0] == '1';
-  const bool want_bn = bn_x != nullptr;
+  const bool want_bn = bn_x != nullptr && bn_coef == nullptr;
   bool fuse_bn = want_bn && epi_bnbwd && !accumulate && d->Cin <= kMaxStatChannels;
   const int s = d->stride;
   const int taps_total = d->KH * d->KW;
@@ -704,6 +726,14 @@ static int32_t dgrad_impl(const T2RConvDesc* d, const void* dy, const void* w_dg
       p.out = out;
       p.residual = accumulate ? out : nullptr;
       p.flags = accumulate ? T2R_EPI_RESIDUAL : 0;
+      if (bn_coef != nullptr) {   // t2r_conv2d_dgrad_bnapply: one phase, one tap, TMA epilogue (checked there)
+        p.flags = kEpiBnApply;
+        p.bn_x = bn_x;
+        p.bn_scale = bn_scale;
+        p.bn_shift = bn_shift;
+        p.bn_coef = bn_coef;
+        p.residual = dpass;
+      }
       if (fuse_bn) {
         p.flags |= kEpiBnBwd;
         p.bn_x = static_cast<const char*>(bn_x) + view_off;

@@ -26,19 +26,25 @@ struct IgemmTmaParams {
   IgemmParams g;
   CUtensorMap tmap_c;  // output view, box 64 x TW x TH x 1
   CUtensorMap tmap_r;  // residual, same geometry
+  CUtensorMap tmap_x;  // kEpiBnApply: the batch-norm input x, same geometry
 };
 
-template <int BLOCK_N>
+// kApply (kEpiBnApply): x lands in the C buffer (the output overwrites it in place) and the residual in a second
+// pair of buffers; no column sums.  The GEMMs it serves have K = 64-256 (1-4 k-iterations per tile), so fewer
+// operand stages make room for the extra buffers.
+template <int BLOCK_N, bool kApply = false>
 struct IgemmTmaCfg {
   static constexpr int kABytes = 128 * 128;
   static constexpr int kBBytes = BLOCK_N * 128;
   static constexpr int kStageBytes = kABytes + kBBytes;
-  static constexpr int kStages = BLOCK_N == 64 ? 6 : 4;
+  static constexpr int kStages = BLOCK_N == 64 ? 6 : (kApply ? 3 : 4);
   static constexpr int kSubTiles = BLOCK_N / 64;
   static constexpr int kCBytes = kSubTiles * 128 * 128;  // one bf16 output tile
+  static constexpr int kRBytes = kApply ? 2 * kCBytes : 0;
   static constexpr int kTmemCols = 2 * BLOCK_N;
-  static constexpr int kStatBytes = 2 * kMaxStatChannels * 4;
-  static constexpr int kSmemBytes = kStages * kStageBytes + 2 * kCBytes + kStatBytes + 256 + 1024;
+  static constexpr int kStatBytes = kApply ? 0 : 2 * kMaxStatChannels * 4;
+  static constexpr int kSmemBytes = kStages * kStageBytes + 2 * kCBytes + kRBytes + kStatBytes + 256 + 1024;
+  static_assert(kSmemBytes <= 232448, "shared memory");
 };
 
 __device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, uint32_t src, int c0, int c1, int c2, int c3) {
@@ -52,16 +58,18 @@ __device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, uint32_t sr
 // residual traffic, and two consecutive tiles' epilogues run on the same warps: with 8 warps each converts two
 // 32-column chunks per tile (~2 x 900 cycles of dependent TMEM load -> shared load -> convert -> shared store ->
 // column sums) and the tile rate is latency bound at ~0.6 of the HBM roofline; 16 warps take one chunk each.
-template <int BLOCK_N, bool kPro, int kEpiWarps>
+template <int BLOCK_N, bool kPro, int kEpiWarps, bool kApply>
 __global__ void __launch_bounds__(128 + 32 * kEpiWarps + (kPro ? 128 : 0), 1)
 conv_igemm_tma_kernel(const __grid_constant__ IgemmTmaParams pp) {
   static_assert(kEpiWarps == 8 || (kEpiWarps == 16 && BLOCK_N == 128 && !kPro), "16 epilogue warps: BLOCK_N 128 only");
-  using Cfg = IgemmTmaCfg<BLOCK_N>;
+  static_assert(!(kPro && kApply), "operand transform and batch-norm apply epilogue do not combine");
+  using Cfg = IgemmTmaCfg<BLOCK_N, kApply>;
   const IgemmParams& p = pp.g;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t c_base = smem_base + Cfg::kStages * Cfg::kStageBytes;
-  const uint32_t stat_base = c_base + 2 * Cfg::kCBytes;
+  const uint32_t r_base = c_base + 2 * Cfg::kCBytes;   // kApply: residual tiles
+  const uint32_t stat_base = r_base + Cfg::kRBytes;
   const uint32_t bar_base = stat_base + Cfg::kStatBytes;
   auto full_bar = [&](int s) { return bar_base + 8u * s; };
   auto empty_bar = [&](int s) { return bar_base + 8u * (Cfg::kStages + s); };
@@ -79,12 +87,15 @@ conv_igemm_tma_kernel(const __grid_constant__ IgemmTmaParams pp) {
   const int lane = threadIdx.x & 31;
   const bool bnbwd = (p.flags & kEpiBnBwd) != 0;  // the "residual" tile is then the normalised tensor x
   const bool has_res = (p.flags & T2R_EPI_RESIDUAL) != 0 || bnbwd;
+  const bool apply_res = kApply && p.residual != nullptr;
+  const bool loads_c = has_res || kApply;             // warp 3 feeds the C buffers
 
   if (warp == 0 && lane == 0) {
     for (int i = 0; i < 4; ++i) tma_prefetch_desc(&p.tmap_a[i]);
     tma_prefetch_desc(&p.tmap_b);
     tma_prefetch_desc(&pp.tmap_c);
     tma_prefetch_desc(&pp.tmap_r);
+    if (kApply) tma_prefetch_desc(&pp.tmap_x);
   }
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < Cfg::kStages; ++s) {
@@ -121,7 +132,7 @@ conv_igemm_tma_kernel(const __grid_constant__ IgemmTmaParams pp) {
     // never waits for an output store.
     if (lane == 0) {
       const int pid = warp == 0 ? 0 : warp - 1;
-      const int n_prod = has_res ? 2 : 3;
+      const int n_prod = loads_c ? 2 : 3;
       if (pid < n_prod) {
         int stage = 0, turn = 0;
         uint32_t phase = 0;
@@ -161,11 +172,16 @@ conv_igemm_tma_kernel(const __grid_constant__ IgemmTmaParams pp) {
           const int oh0 = (rem / p.tiles_w) * p.TH;
           const int ow0 = (rem % p.tiles_w) * p.TW;
           mbar_wait(cempty_bar(cb), cphase ^ 1u);  // the store that last used this buffer has read it
-          mbar_expect_tx(cfull_bar(cb), Cfg::kCBytes);
+          mbar_expect_tx(cfull_bar(cb), apply_res ? 2 * Cfg::kCBytes : Cfg::kCBytes);
 #pragma unroll
           for (int j = 0; j < Cfg::kSubTiles; ++j)
-            tma_load_4d(c_base + cb * Cfg::kCBytes + j * 16384, &pp.tmap_r, cfull_bar(cb), nt * BLOCK_N + j * 64, ow0,
-                        oh0, img);
+            tma_load_4d(c_base + cb * Cfg::kCBytes + j * 16384, kApply ? &pp.tmap_x : &pp.tmap_r, cfull_bar(cb),
+                        nt * BLOCK_N + j * 64, ow0, oh0, img);
+          if (apply_res)
+#pragma unroll
+            for (int j = 0; j < Cfg::kSubTiles; ++j)
+              tma_load_4d(r_base + cb * Cfg::kCBytes + j * 16384, &pp.tmap_r, cfull_bar(cb), nt * BLOCK_N + j * 64, ow0,
+                          oh0, img);
           if (++cb == 2) {
             cb = 0;
             cphase ^= 1u;
@@ -263,12 +279,13 @@ conv_igemm_tma_kernel(const __grid_constant__ IgemmTmaParams pp) {
       const bool valid = (oh0 + th < p.Ho) && (ow0 + tw < p.Wo);
       const uint32_t csub = c_base + cb * Cfg::kCBytes + sub * 16384;
       const uint32_t crow = csub + uint32_t(row) * 128u;
+      const uint32_t rrow = crow + (r_base - c_base);   // kApply: the residual row beside it
       if (elected && pending_cb >= 0) {
         asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
         mbar_arrive(cempty_bar(pending_cb));
         pending_cb = -1;
       }
-      if (has_res) mbar_wait(cfull_bar(cb), cphase);   // the residual tile has landed in the C buffer
+      if (loads_c) mbar_wait(cfull_bar(cb), cphase);   // the residual tile has landed in the C buffer
       else mbar_wait(cempty_bar(cb), cphase ^ 1u);     // the store that last used the buffer has read it
       mbar_wait(tfull_bar(as), aphase);
       tc_fence_after();
@@ -290,7 +307,39 @@ conv_igemm_tma_kernel(const __grid_constant__ IgemmTmaParams pp) {
           }
         }
         const uint32_t chunk0 = uint32_t(colc) >> 3;          // first 16-byte chunk of these 32 columns
-        if (bnbwd) {
+        if (kApply) {
+          // dx = scale * [scale * x + shift > 0] * acc + kb * x + kc (+ residual); the arithmetic of
+          // bn_bwd_apply_kernel (norm.cu) on the fp32 accumulator instead of the bf16-rounded g
+#pragma unroll
+          for (uint32_t j = 0; j < 4; ++j) {
+            const uint32_t off = ((chunk0 + j) ^ rsw) << 4;
+            uint4 q, r = make_uint4(0u, 0u, 0u, 0u);
+            asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];"
+                         : "=r"(q.x), "=r"(q.y), "=r"(q.z), "=r"(q.w)
+                         : "r"(crow + off)
+                         : "memory");
+            if (apply_res)
+              asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];"
+                           : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
+                           : "r"(rrow + off)
+                           : "memory");
+            const uint32_t qv[4] = {q.x, q.y, q.z, q.w}, rv[4] = {r.x, r.y, r.z, r.w};
+            float sc[8], sh[8], kb[8], kc[8];
+            const int c8 = ch + 8 * int(j);
+            load8(p.bn_scale + c8, sc);
+            load8(p.bn_shift + c8, sh);
+            load8(p.bn_coef + c8, kb);
+            load8(p.bn_coef + p.Cout + c8, kc);
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+              const float x = (i & 1) ? bf16_hi(qv[i >> 1]) : bf16_lo(qv[i >> 1]);
+              const float dz = fmaf(x, sc[i], sh[i]) > 0.f ? f[8 * j + i] : 0.f;
+              float o = fmaf(sc[i], dz, fmaf(kb[i], x, kc[i]));
+              if (apply_res) o += (i & 1) ? bf16_hi(rv[i >> 1]) : bf16_lo(rv[i >> 1]);
+              f[8 * j + i] = o;
+            }
+          }
+        } else if (bnbwd) {
           // g = dz * [scale * x + shift > 0] (x = the tile warp 3 loaded), rounded to bf16 like the stored value;
           // column sums of g * x by shuffles, those of g from the staged tile below (as the fused bn_stats)
           float xv[32];
@@ -412,22 +461,24 @@ conv_igemm_tma_kernel(const __grid_constant__ IgemmTmaParams pp) {
   }
 }
 
-template <int BLOCK_N, bool kPro, int kEpiWarps>
+template <int BLOCK_N, bool kPro, int kEpiWarps, bool kApply = false>
 static int launch_v(const IgemmTmaParams& pp, cudaStream_t stream) {
-  using Cfg = IgemmTmaCfg<BLOCK_N>;
+  using Cfg = IgemmTmaCfg<BLOCK_N, kApply>;
   static bool configured = false;
   if (!configured) {
-    T2R_CUDA_OK(cudaFuncSetAttribute(conv_igemm_tma_kernel<BLOCK_N, kPro, kEpiWarps>,
+    T2R_CUDA_OK(cudaFuncSetAttribute(conv_igemm_tma_kernel<BLOCK_N, kPro, kEpiWarps, kApply>,
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
     configured = true;
   }
   const int grid = std::min(pp.g.total_tiles, num_sms());
-  conv_igemm_tma_kernel<BLOCK_N, kPro, kEpiWarps><<<grid, 128 + 32 * kEpiWarps + (kPro ? 128 : 0), Cfg::kSmemBytes, stream>>>(pp);
+  conv_igemm_tma_kernel<BLOCK_N, kPro, kEpiWarps, kApply>
+      <<<grid, 128 + 32 * kEpiWarps + (kPro ? 128 : 0), Cfg::kSmemBytes, stream>>>(pp);
   T2R_LAUNCH_OK();
   return T2R_OK;
 }
 template <int BLOCK_N>
 static int launch(const IgemmTmaParams& pp, cudaStream_t stream) {
+  if (pp.g.flags & kEpiBnApply) return launch_v<BLOCK_N, false, 8, true>(pp, stream);
   if (pp.g.flags & kProBnRelu) return launch_v<BLOCK_N, true, 8>(pp, stream);
   return launch_v<BLOCK_N, false, 8>(pp, stream);
 }
@@ -436,6 +487,7 @@ static int launch(const IgemmTmaParams& pp, cudaStream_t stream) {
 // 142.6 -> 143.5 ms), so 8 stays the default - the low-K layers are not bound by the epilogue's latency.
 template <>
 int launch<128>(const IgemmTmaParams& pp, cudaStream_t stream) {
+  if (pp.g.flags & kEpiBnApply) return launch_v<128, false, 8, true>(pp, stream);
   if (pp.g.flags & kProBnRelu) return launch_v<128, true, 8>(pp, stream);
   static const char* mode = std::getenv("T2R_TMA_EPI_WARPS");
   const int k_iters = pp.g.n_taps * pp.g.chunks_per_tap;
@@ -455,6 +507,8 @@ int conv_igemm_tma_launch(const IgemmParams& p, int block_n, cudaStream_t stream
   if (encode_tmap_bf16(&pp.tmap_c, p.out, 4, dims, strides, box) != 0) return T2R_ERR_CUDA;
   const void* aux = (p.flags & kEpiBnBwd) ? p.bn_x : p.residual;
   if (encode_tmap_bf16(&pp.tmap_r, aux ? aux : p.out, 4, dims, strides, box) != 0) return T2R_ERR_CUDA;
+  pp.tmap_x = pp.tmap_r;
+  if ((p.flags & kEpiBnApply) && encode_tmap_bf16(&pp.tmap_x, p.bn_x, 4, dims, strides, box) != 0) return T2R_ERR_CUDA;
   return block_n == 128 ? launch<128>(pp, stream) : launch<64>(pp, stream);
 }
 

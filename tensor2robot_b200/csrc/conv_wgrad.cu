@@ -48,7 +48,47 @@ struct WgradParams {
   // X tile as relu(bn_scale * x + bn_shift) before the MMA reads it (see kProBnRelu, conv_common.cuh)
   const float* bn_scale;
   const float* bn_shift;
+  // kBnSums: 1x1 consumer of z = relu(bn_scale * x + bn_shift), x raw.  A group is ONE 64-channel chunk c: the
+  // transform warps rewrite its landed x tile as m * x and write m = [bn_scale * x + bn_shift > 0] into the second
+  // A slot, so that TMEM rows 0-63 hold P[c, n] = sum dy * m * x and rows 64-127 Q[c, n] = sum dy * m.  The epilogue
+  // adds dw[n, c] += bn_scale * P + bn_shift * Q (= sum dy * z) and bn_sums[c] += sum_n w[c, n] * Q (= sum g),
+  // bn_sums[Cin + c] += sum_n w[c, n] * P (= sum g * x), g = m * (dy conv_transpose w): the batch-norm reduction
+  // without a pass over g.  w_dgrad: the bf16 [Cin][Cout] weights the data gradient multiplies with.
+  const uint16_t* w_dgrad;
+  double* bn_sums;
 };
+
+enum WgradMode { kWgPlain = 0, kWgBnRelu = 1, kWgBnSums = 2 };
+
+// kWgBnSums operand transform on kN 16-byte pieces (8 channels, `step` bytes apart) of a SW128 x tile: x -> m * x in
+// place and m (bf16 1.0 / 0.0) at the same position `mask_off` bytes further.  Both are exact in bf16; the mask test
+// is the fmaf of bn_bwd_reduce_kernel (norm.cu).
+template <int kN>
+__device__ __forceinline__ void bnmask_pieces(uint32_t piece, uint32_t step, uint32_t mask_off, const float (&sc)[8],
+                                              const float (&sh)[8]) {
+  uint4 q[kN];
+#pragma unroll
+  for (int i = 0; i < kN; ++i)
+    asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];"
+                 : "=r"(q[i].x), "=r"(q[i].y), "=r"(q[i].z), "=r"(q[i].w)
+                 : "r"(piece + uint32_t(i) * step)
+                 : "memory");
+#pragma unroll
+  for (int i = 0; i < kN; ++i) {
+    uint32_t w[4] = {q[i].x, q[i].y, q[i].z, q[i].w}, keep[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k)
+      keep[k] = (fmaf(bf16_lo(w[k]), sc[2 * k], sh[2 * k]) > 0.f ? 0x0000FFFFu : 0u) |
+                (fmaf(bf16_hi(w[k]), sc[2 * k + 1], sh[2 * k + 1]) > 0.f ? 0xFFFF0000u : 0u);
+    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(piece + uint32_t(i) * step), "r"(w[0] & keep[0]),
+                 "r"(w[1] & keep[1]), "r"(w[2] & keep[2]), "r"(w[3] & keep[3])
+                 : "memory");
+    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(piece + uint32_t(i) * step + mask_off),
+                 "r"(keep[0] & 0x3F803F80u), "r"(keep[1] & 0x3F803F80u), "r"(keep[2] & 0x3F803F80u),
+                 "r"(keep[3] & 0x3F803F80u)
+                 : "memory");
+  }
+}
 
 template <int BLOCK_N>
 struct WgradCfg {
@@ -62,9 +102,11 @@ struct WgradCfg {
   static constexpr int kSmemBytes = kXStages * kXBytes + kDyStages * kDyBytes + 1024 + 512;
 };
 
-template <int BLOCK_N, bool kPro>
+template <int BLOCK_N, int kMode>
 __global__ void __launch_bounds__(256, 1) conv_wgrad_kernel(const __grid_constant__ WgradParams p) {
   using Cfg = WgradCfg<BLOCK_N>;
+  constexpr bool kPro = kMode != kWgPlain;   // the epilogue warps transform the landed X tiles
+  constexpr bool kSums = kMode == kWgBnSums;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t dy_base = smem_base + Cfg::kXStages * Cfg::kXBytes;
@@ -150,9 +192,10 @@ __global__ void __launch_bounds__(256, 1) conv_wgrad_kernel(const __grid_constan
           if (turn == pid) {
             mbar_wait(empty_bar(stage), phase ^ 1u);
             const uint32_t sa = smem_base + stage * Cfg::kXBytes;
-            mbar_expect_tx(full_bar(stage), Cfg::kXBytes);
+            mbar_expect_tx(full_bar(stage), kSums ? Cfg::kTileBytes : Cfg::kXBytes);
+            if (kSums) tma_load_4d(sa, &p.tmap_x[0], full_bar(stage), g * 64, ow0, oh0, img);
 #pragma unroll
-            for (int h = 0; h < 2; ++h) {
+            for (int h = 0; h < (kSums ? 0 : 2); ++h) {
               int slot = 2 * g + h;
               if (slot >= p.n_slots) slot = p.n_slots - 1;  // duplicate: rows are never stored
               const int t = slot / p.chunks_per_tap;
@@ -207,7 +250,29 @@ __global__ void __launch_bounds__(256, 1) conv_wgrad_kernel(const __grid_constan
   } else if (warp >= 4) {
     const int quad = warp - 4;
     const int row = quad * 32 + lane;
-    if (kPro) {
+    if (kSums) {
+      // operand transform: 128 threads over the 64 rows x 8 chunks of the group's x tile, 4 rows r0 + 16 i each
+      const int t = threadIdx.x - 128;
+      const uint32_t j = uint32_t(t) & 7u, r0 = uint32_t(t) >> 3;
+      const uint32_t piece0 = r0 * 128u + ((j ^ (r0 & 7u)) << 4);
+      int stage = 0;
+      uint32_t phase = 0;
+      for (int pt = pt0; pt < pt1; ++pt)
+        for (int g = g0; g < g1; ++g) {
+          float sc[8], sh[8];
+          load8(p.bn_scale + g * 64 + j * 8, sc);
+          load8(p.bn_shift + g * 64 + j * 8, sh);
+          mbar_wait(full_bar(stage), phase);
+          bnmask_pieces<4>(smem_base + stage * Cfg::kXBytes + piece0, 2048u, Cfg::kTileBytes, sc, sh);
+          fence_proxy_async_smem();
+          __syncwarp();
+          if (lane == 0) mbar_arrive(ready_bar(stage));
+          if (++stage == Cfg::kXStages) {
+            stage = 0;
+            phase ^= 1u;
+          }
+        }
+    } else if (kPro) {
       // operand transform: thread t works on tile h = t / 64 of the stage (64 rows x 128 B), logical chunk t & 7 of
       // rows ((t & 63) >> 3) + 8 i: a quarter warp covers one full row, a thread's rows share r & 7
       const int t = threadIdx.x - 128;
@@ -235,7 +300,45 @@ __global__ void __launch_bounds__(256, 1) conv_wgrad_kernel(const __grid_constan
           }
         }
     }
-    if (pt1 > pt0) {
+    if (kSums && pt1 > pt0) {
+      // Thread `row` holds P (rows 0-63) or Q (rows 64-127) of channel c = row & 63.  Both halves go through shared
+      // memory (the idle X ring, double-buffered so one barrier per 32 columns suffices); each thread then finishes
+      // 16 of the 32 columns of its channel.
+      mbar_wait(tfull_bar, 0);
+      tc_fence_after();
+      float* xch = reinterpret_cast<float*>(smem_raw + (smem_base - smem_u32(smem_raw)));
+      const int c = row & 63, jh = (row >> 6) * 16;
+      int b = 0;
+      for (int g = g0; g < g1; ++g) {
+        const int k = g * 64 + c;
+        const float sc = p.bn_scale[k], sh = p.bn_shift[k];
+        float s_p = 0.f, s_q = 0.f;
+#pragma unroll 1
+        for (int c0 = 0; c0 < BLOCK_N; c0 += 32, b ^= 1) {
+          uint32_t v[32];
+          tmem_ld_32x32(tmem_base + (uint32_t(quad * 32) << 16) + (g - g0) * BLOCK_N + c0, v);
+          tmem_ld_wait();
+          float* buf = xch + b * 4096;   // [P | Q][32 columns][64 channels]
+#pragma unroll
+          for (int j = 0; j < 32; ++j) buf[((row >> 6) * 32 + j) * 64 + c] = __uint_as_float(v[j]);
+          asm volatile("bar.sync 1, 128;" ::: "memory");
+          const uint4* wp = reinterpret_cast<const uint4*>(p.w_dgrad + (long long)k * p.Cout + n0 + c0 + jh);
+          const uint4 w0 = __ldg(wp), w1 = __ldg(wp + 1);
+          const uint32_t wv[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
+          float* dst = p.dw + (long long)(n0 + c0 + jh) * p.Ktot + k;
+#pragma unroll
+          for (int jj = 0; jj < 16; ++jj) {
+            const float pv = buf[(jh + jj) * 64 + c], qv = buf[(32 + jh + jj) * 64 + c];
+            const float w = (jj & 1) ? bf16_hi(wv[jj >> 1]) : bf16_lo(wv[jj >> 1]);
+            atomicAdd(dst + (long long)jj * p.Ktot, fmaf(sc, pv, sh * qv));
+            s_p = fmaf(w, pv, s_p);
+            s_q = fmaf(w, qv, s_q);
+          }
+        }
+        atomicAdd(p.bn_sums + k, double(s_q));
+        atomicAdd(p.bn_sums + p.Ktot + k, double(s_p));
+      }
+    } else if (pt1 > pt0) {
       mbar_wait(tfull_bar, 0);
       tc_fence_after();
       for (int g = g0; g < g1; ++g) {
@@ -272,12 +375,12 @@ static int launch_wgrad(WgradParams& p, cudaStream_t stream) {
   using Cfg = WgradCfg<BLOCK_N>;
   static bool configured = false;
   if (!configured) {
-    T2R_CUDA_OK(cudaFuncSetAttribute(conv_wgrad_kernel<BLOCK_N, false>,
-                                     cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     Cfg::kSmemBytes));
-    T2R_CUDA_OK(cudaFuncSetAttribute(conv_wgrad_kernel<BLOCK_N, true>,
-                                     cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     Cfg::kSmemBytes));
+    T2R_CUDA_OK(cudaFuncSetAttribute(conv_wgrad_kernel<BLOCK_N, kWgPlain>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
+    T2R_CUDA_OK(cudaFuncSetAttribute(conv_wgrad_kernel<BLOCK_N, kWgBnRelu>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
+    T2R_CUDA_OK(cudaFuncSetAttribute(conv_wgrad_kernel<BLOCK_N, kWgBnSums>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
     configured = true;
   }
   p.groups_per_cta = std::min(p.n_groups, Cfg::kMaxGroups);
@@ -291,10 +394,12 @@ static int launch_wgrad(WgradParams& p, cudaStream_t stream) {
   ks = std::max(1, std::min(ks, std::max(1, p.total_ptiles / 4)));
   p.ksplits = ks;
   const int grid = base_items * ks;
-  if (p.bn_scale != nullptr)
-    conv_wgrad_kernel<BLOCK_N, true><<<grid, 256, Cfg::kSmemBytes, stream>>>(p);
+  if (p.bn_sums != nullptr)
+    conv_wgrad_kernel<BLOCK_N, kWgBnSums><<<grid, 256, Cfg::kSmemBytes, stream>>>(p);
+  else if (p.bn_scale != nullptr)
+    conv_wgrad_kernel<BLOCK_N, kWgBnRelu><<<grid, 256, Cfg::kSmemBytes, stream>>>(p);
   else
-    conv_wgrad_kernel<BLOCK_N, false><<<grid, 256, Cfg::kSmemBytes, stream>>>(p);
+    conv_wgrad_kernel<BLOCK_N, kWgPlain><<<grid, 256, Cfg::kSmemBytes, stream>>>(p);
   T2R_LAUNCH_OK();
   return T2R_OK;
 }
@@ -304,11 +409,11 @@ static int launch_wgrad(WgradParams& p, cudaStream_t stream) {
 using namespace t2r;
 
 static int32_t wgrad_impl(const T2RConvDesc* d, const void* x, const float* bn_scale, const float* bn_shift,
-                          const void* dy, float* dw, void* stream);
+                          const void* dy, float* dw, const void* w_dgrad, double* bn_sums, void* stream);
 
 extern "C" int32_t t2r_conv2d_wgrad(const T2RConvDesc* d, const void* x, const void* dy,
                                     float* dw, void* stream) {
-  return wgrad_impl(d, x, nullptr, nullptr, dy, dw, stream);
+  return wgrad_impl(d, x, nullptr, nullptr, dy, dw, nullptr, nullptr, stream);
 }
 
 extern "C" int32_t t2r_conv2d_wgrad_bnrelu(const T2RConvDesc* d, const void* x_raw, const float* bn_scale,
@@ -317,11 +422,21 @@ extern "C" int32_t t2r_conv2d_wgrad_bnrelu(const T2RConvDesc* d, const void* x_r
   T2R_CHECK_ARG(bn_scale && bn_shift, "conv2d_wgrad_bnrelu: null scale / shift");
   T2R_CHECK_ARG(d->KH == 1 && d->KW == 1 && d->pad_top == 0 && d->pad_left == 0,
                 "conv2d_wgrad_bnrelu: only 1x1 convolutions without padding fuse the batch-norm apply");
-  return wgrad_impl(d, x_raw, bn_scale, bn_shift, dy, dw, stream);
+  return wgrad_impl(d, x_raw, bn_scale, bn_shift, dy, dw, nullptr, nullptr, stream);
+}
+
+extern "C" int32_t t2r_conv2d_wgrad_bnsums(const T2RConvDesc* d, const void* x_raw, const float* bn_scale,
+                                           const float* bn_shift, const void* dy, const void* w_dgrad, float* dw,
+                                           double* bn_sums, void* stream) {
+  T2R_CHECK_ARG(d != nullptr && d->struct_size == sizeof(T2RConvDesc), "bad T2RConvDesc size");
+  T2R_CHECK_ARG(bn_scale && bn_shift && w_dgrad && bn_sums, "conv2d_wgrad_bnsums: null pointer");
+  T2R_CHECK_ARG(d->KH == 1 && d->KW == 1 && d->stride == 1 && d->pad_top == 0 && d->pad_left == 0,
+                "conv2d_wgrad_bnsums: 1x1 stride-1 convolutions without padding only");
+  return wgrad_impl(d, x_raw, bn_scale, bn_shift, dy, dw, w_dgrad, bn_sums, stream);
 }
 
 static int32_t wgrad_impl(const T2RConvDesc* d, const void* x, const float* bn_scale, const float* bn_shift,
-                          const void* dy, float* dw, void* stream) {
+                          const void* dy, float* dw, const void* w_dgrad, double* bn_sums, void* stream) {
   T2R_CHECK_ARG(d != nullptr && d->struct_size == sizeof(T2RConvDesc), "bad T2RConvDesc size");
   T2R_CHECK_ARG(d->stride == 1 || d->stride == 2, "stride must be 1 or 2");
   T2R_CHECK_ARG(d->KH * d->KW <= kMaxTaps, "filter too large");
@@ -348,11 +463,11 @@ static int32_t wgrad_impl(const T2RConvDesc* d, const void* x, const float* bn_s
       p.taps[t].dw = int8_t(floor_div(iw, d->stride));
       p.taps[t].kchunk0 = t * p.chunks_per_tap;
     }
-  if (conv_wgrad_halo_eligible(d->stride, t, d->Cin, d->Cout))
+  if (bn_sums == nullptr && conv_wgrad_halo_eligible(d->stride, t, d->Cin, d->Cout))
     return conv_wgrad_halo_launch(x, dy, dw, d->N, d->H, d->W, d->Ho, d->Wo, d->Cout, p.taps, t,
                                   static_cast<cudaStream_t>(stream));
   p.n_slots = t * p.chunks_per_tap;
-  p.n_groups = (p.n_slots + 1) / 2;
+  p.n_groups = bn_sums != nullptr ? p.n_slots : (p.n_slots + 1) / 2;
   p.tiles_w = int(ceil_div(d->Wo, p.TW));
   p.tiles_h = int(ceil_div(d->Ho, p.TH));
   p.total_ptiles = d->N * p.tiles_w * p.tiles_h;
@@ -361,6 +476,8 @@ static int32_t wgrad_impl(const T2RConvDesc* d, const void* x, const float* bn_s
   p.dw = dw;
   p.bn_scale = bn_scale;
   p.bn_shift = bn_shift;
+  p.w_dgrad = static_cast<const uint16_t*>(w_dgrad);
+  p.bn_sums = bn_sums;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (d->Cout % 256 == 0) return launch_wgrad<256>(p, st);
   if (d->Cout % 128 == 0) return launch_wgrad<128>(p, st);

@@ -220,6 +220,22 @@ __global__ void bn_bwd_finalize_kernel(const double* red, int C, const float* me
   dgamma[c] = float((red[C + c] - double(mean[c]) * red[c]) * double(invstd[c]));
 }
 
+// t2r_bn_backward_gemm_finalize: sums[c] = sum g, sums[C + c] = sum g * x from t2r_conv2d_wgrad_bnsums.  Writes
+// dgamma / dbeta as bn_bwd_finalize_kernel and the apply coefficients kb, kc of bn_bwd_apply_kernel into coef [2C].
+__global__ void bn_bwd_gemm_finalize_kernel(const double* sums, int C, float inv_rows, const float* mean,
+                                            const float* invstd, const float* scale, float* dgamma, float* dbeta,
+                                            float* coef) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  const float db = float(sums[c]);
+  const float dg = float((sums[C + c] - double(mean[c]) * sums[c]) * double(invstd[c]));
+  dbeta[c] = db;
+  dgamma[c] = dg;
+  const float t = scale[c] * dg * inv_rows * invstd[c];
+  coef[c] = -t;
+  coef[C + c] = t * mean[c] - scale[c] * db * inv_rows;
+}
+
 // pass 2: dx = scale * (dz - sum(dz)/rows - xhat * sum(dz*xhat)/rows) (+ dres)
 //            = scale*dz + kb*x + kc   with per-channel kb, kc.
 // Row-partitioned like the reductions: a thread owns one 8-channel group, so the coefficients
@@ -523,6 +539,17 @@ extern "C" int32_t t2r_bn_backward_presummed(const void* dy, const void* x, cons
     bn_bwd_apply_kernel<false><<<grid, 256, 0, st>>>(
         static_cast<const uint4*>(dy), static_cast<const uint4*>(x), nullptr, static_cast<uint4*>(dx), rows, C,
         p.cgb, p.lanes_r, p.rows_per_block, inv_rows, mean, invstd, scale, shift, dgamma, dbeta, relu);
+  T2R_LAUNCH_OK();
+  return T2R_OK;
+}
+
+extern "C" int32_t t2r_bn_backward_gemm_finalize(const double* sums, int64_t rows, int32_t C, const float* mean,
+                                                 const float* invstd, const float* scale, float* dgamma, float* dbeta,
+                                                 float* coef, void* stream) {
+  T2R_CHECK_ARG(sums && mean && invstd && scale && dgamma && dbeta && coef, "bn_backward_gemm_finalize: null pointer");
+  T2R_CHECK_ARG(rows > 0 && C > 0, "bn_backward_gemm_finalize: bad shape");
+  bn_bwd_gemm_finalize_kernel<<<(C + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(
+      sums, C, 1.f / float(rows), mean, invstd, scale, dgamma, dbeta, coef);
   T2R_LAUNCH_OK();
   return T2R_OK;
 }

@@ -553,11 +553,25 @@ FOLD_INFERENCE_BN = os.environ.get('T2R_FOLD_INFERENCE_BN', '1') != '0'
 #   * masked / reduced data gradients (t2r_conv2d_dgrad_bnrelu): correct and tested, but the epilogue needs ~24
 #     instructions per element against a budget of ~6 at HBM speed, so the stand-alone reduction pass is faster
 #     (same file); the C entry point therefore fuses only when T2R_BNBWD_EPI=1.
-# T2R_FUSE_BN_NODE=0 restores the separate nodes; T2R_FUSE_BN_OPERAND = 0 | auto | all.
+#   * backward through the consumer's GEMMs (_bn_bwd_gemm_eligible): when the only consumer is a 1x1 stride-1
+#     convolution whose data gradient runs on the TMA-epilogue kernel, its weight gradient also yields the two
+#     batch-norm sums (t2r_conv2d_wgrad_bnsums) and its data gradient writes dx itself (t2r_conv2d_dgrad_bnapply):
+#     g, the reduction pass and the apply pass disappear, and z is not kept for backward.
+# T2R_FUSE_BN_NODE=0 restores the separate nodes; T2R_FUSE_BN_OPERAND = 0 | auto | all; T2R_BN_BWD_GEMM=0 restores
+# the data gradient + reduction + apply backward everywhere.
 FUSE_BN_NODE = os.environ.get('T2R_FUSE_BN_NODE', '1') != '0'
 FUSE_BN_OPERAND = os.environ.get('T2R_FUSE_BN_OPERAND', 'auto')
 _BN_OPERAND_MAX_COUT = int(os.environ.get('T2R_BN_OPERAND_MAX_COUT', '128'))
 FUSE_BN_BWD_EPILOGUE = os.environ.get('T2R_BNBWD_EPI', '0') == '1'
+BN_BWD_GEMM = os.environ.get('T2R_BN_BWD_GEMM', '1') != '0'
+
+
+def _bn_bwd_gemm_eligible(convs, descs):
+  if not BN_BWD_GEMM or len(convs) != 1:
+    return False
+  var = convs[0][0]
+  return (var.trainable and var.dgrad is not None
+          and _lib.lib().t2r_conv2d_dgrad_bnapply_supported(C.byref(descs[0])) == 1)
 
 
 def _bn_operand_fusable(cin, cout, kh, kw, pt, pl, has_res):
@@ -853,7 +867,8 @@ class _BnReluConvFn(torch.autograd.Function):
       descs.append(d)
     ctx.bn, ctx.vs, ctx.descs, ctx.vars = bn, vs, descs, [cv[0] for cv in convs]
     ctx.operand_fused, ctx.passthrough, ctx.has_res = operand_fused, passthrough, residual is not None
-    ctx.save_for_backward(x, mean, invstd, scale, shift, z)
+    ctx.bwd_gemm = ctx.needs_input_grad[0] and _bn_bwd_gemm_eligible(convs, descs)
+    ctx.save_for_backward(x, mean, invstd, scale, shift, None if ctx.bwd_gemm else z)
     if passthrough:
       outs.append(x.view_as(x))
     return tuple(outs)
@@ -869,6 +884,8 @@ class _BnReluConvFn(torch.autograd.Function):
     if dpass is not None:
       dpass = dpass.contiguous()
     dys = [g.contiguous() if g is not None else None for g in grads[:len(ctx.vars)]]
+    if ctx.bwd_gemm and dys[0] is not None:
+      return _BnReluConvFn._backward_gemm(ctx, x, mean, invstd, scale, shift, dys[0], dpass)
     for var, d, dy in zip(ctx.vars, ctx.descs, dys):
       if dy is None or not var.trainable:
         continue
@@ -908,6 +925,33 @@ class _BnReluConvFn(torch.autograd.Function):
                   _p(mean), _p(invstd), _p(scale), _p(shift), 1, _p(red), _p(dgamma), _p(dbeta), st)
       _bn_grads_ready(bn)
     dres = dys[0] if (ctx.has_res and ctx.needs_input_grad[1]) else None
+    return dx, dres, None, None, None, None, None, None
+
+  @staticmethod
+  def _backward_gemm(ctx, x, mean, invstd, scale, shift, dy, dpass):
+    """Single 1x1 consumer: dual-operand weight gradient (dw and the two batch-norm sums), finalize (dgamma, dbeta
+    and the apply coefficients), data gradient whose epilogue writes dx."""
+    bn, vs, var, d = ctx.bn, ctx.vs, ctx.vars[0], ctx.descs[0]
+    c = x.shape[-1]
+    rows = x.numel() // c
+    st = _stream()
+    sums = torch.zeros(2 * c, dtype=torch.float64, device=x.device)
+    coef = torch.empty(2 * c, dtype=F32, device=x.device)
+    with _prof('wgrad', d):
+      _lib.call('t2r_conv2d_wgrad_bnsums', C.byref(d), _p(x), _p(scale), _p(shift), _p(dy), _p(var.dgrad),
+                _p(var.grad), _p(sums), st)
+    var.grad_ready()
+    gamma = bn['gamma']
+    dgamma = gamma.grad if (gamma is not None and gamma.trainable) else vs.scratch('bn_dgamma', 4096, F32)
+    dbeta = bn['beta'].grad if bn['beta'].trainable else vs.scratch('bn_dbeta', 4096, F32)
+    _lib.call('t2r_bn_backward_gemm_finalize', _p(sums), rows, c, _p(mean), _p(invstd), _p(scale), _p(dgamma),
+              _p(dbeta), _p(coef), st)
+    _bn_grads_ready(bn)
+    dx = torch.empty_like(x)
+    with _prof('dgrad', d):
+      _lib.call('t2r_conv2d_dgrad_bnapply', C.byref(d), _p(dy), _p(var.dgrad), _p(x), _p(scale), _p(shift), _p(coef),
+                _p(dpass), _p(dx), st)
+    dres = dy if (ctx.has_res and ctx.needs_input_grad[1]) else None
     return dx, dres, None, None, None, None, None, None
 
 
